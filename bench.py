@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this implementation
   python bench.py --impl reference ...                            # CPU arm: torch-eager oracle port on host cores
   torchrun --nproc-per-node N bench.py --gpus N ...               # N > 1: tensor parallel (heads / FFN columns)
+  python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs as .npy
 
 Workload (BASELINE.json configs[1]): Llama-3-8B shapes, bf16, pure decode, batch 256, every sequence at
 seq_len 4096, block_size 16, synthetic seeded weights N(0, 0.02) and a KV cache pre-filled with N(0, 1).
@@ -35,6 +36,9 @@ import torch  # noqa: E402
 
 METRIC = "decode_tokens_per_s"
 UNIT = "tokens/s"
+# --dump-outputs: the full logits of the flagship step (256 x 128256) are 131 MB in fp32; a fixed column sample keeps every
+# sequence comparable at 8 MB
+DUMP_LOGIT_COLUMNS = 8192
 
 
 _T0 = time.perf_counter()
@@ -89,7 +93,14 @@ def parse():
     ap.add_argument("--profile-range", type=int, default=0,
                     help="profiling aid: run this many eager decode steps inside cudaProfilerStart/Stop and exit "
                          "(use with ncu --profile-from-start off); prints no bench line")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed: DIR/tokens.npy (the sampled token "
+                         "of every sequence, float64) and DIR/logits_sample.npy (the logits of every sequence at "
+                         f"{DUMP_LOGIT_COLUMNS} fixed, seeded vocabulary columns, float32; not written with a sharded lm_head)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def model_dict(name, layers=0):
@@ -464,6 +475,17 @@ def parity_check(model, mc, ids, sids, lens, n_rows=8, n_seqs=2, tp_rank=0, tp_s
     return res
 
 
+def dump_outputs(out_dir, tokens, logits):
+    """--dump-outputs: `tokens` [B] and, unless None, a fixed column sample of `logits` [B, V] as .npy files under out_dir."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "tokens.npy"), tokens.cpu().numpy().astype(np.float64))
+    if logits is not None:
+        V = logits.shape[1]
+        cols = np.sort(np.random.default_rng(0).choice(V, size=min(V, DUMP_LOGIT_COLUMNS), replace=False))
+        sample = logits.index_select(1, torch.from_numpy(cols).to(logits.device)).float().cpu().numpy()
+        np.save(os.path.join(out_dir, "logits_sample.npy"), sample)
+
+
 # --------------------------------------------------------------------------- GPU arm
 def run_ours(args):
     import torch.distributed as dist
@@ -499,6 +521,9 @@ def run_ours(args):
                                     shard_lm_head=args.shard_lm_head, fuse_rotary_store=args.fuse_rotary_store)
     model = swiftllm_b200.LlamaModel(ec, mc)
     model.load_weights(synthetic_getter(seed=0, std=0.02, device=dev))
+    # set before the decode graph is captured, so that replays leave their logits where post_layer.last_logits points;
+    # a sharded lm_head would have to gather the full logits in every step for that
+    model.post_layer.keep_logits = bool(args.dump_outputs) and not model.post_layer.sharded
     num_blocks = B * blocks_per_seq + 64
     model.init_kvcache_and_swap(num_blocks)
     g = torch.Generator(device=dev); g.manual_seed(1234 + rank)
@@ -569,12 +594,14 @@ def run_ours(args):
             graph["meta"][:B].copy_(graph["tokens"].to(torch.int32))     # next step's ids = sampled tokens, on device
             graph["graph"].replay()
         else:
-            model.forward_async(state["ids"], sids, lens)
+            state["tokens"] = model.forward_async(state["ids"], sids, lens)
 
     for _ in range(max(args.warmup, 3)):
         step_resident()
     ms_val = timed(step_resident, args.steps)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, graph["tokens"] if graph is not None else state["tokens"], model.post_layer.last_logits)
 
     stage("roofline pass (events around every decode-attention launch)")
     # ---- roofline of the dominant kernel (paged decode attention): eager steps with events around each launch

@@ -5,7 +5,7 @@ Executes the UNMODIFIED reference (swiftLLM at /root/reference) on CPU -- Triton
 TRITON_INTERPRET=1, `LlamaModel` under the cuda->cpu shim of `oracle/ref_shim.py` -- on seeded
 inputs and stores inputs + outputs under `tests/golden/*.npz`.  Run in the build container:
 
-    python oracle/gen_golden.py            # re-executes itself with `python -O`
+    python oracle/gen_golden.py [name ...] # re-executes itself with `python -O`; names: GENERATORS below
 
 (`-O` strips the reference's `assert weight.device.type == "cuda"`, weight.py:49, which cannot
 hold on a CPU-only box; nothing else changes.)  Versions are recorded in each file.
@@ -304,15 +304,35 @@ def gen_model(swiftllm):
     save("model_tiny", **arrays)
 
 
-def main():
+def gen_model_config(swiftllm):
+    """The reference's LlamaModelConfig over GQA / MHA / scaled-RoPE / legacy-key configs: every attribute it defines and
+    its KV-slot size per dtype, one JSON record per config."""
+    from swiftllm.model_config import LlamaModelConfig
+    from swiftllm_b200.model_config import LLAMA3_8B
+    base = dict(LLAMA3_8B)
+    cfgs = [base, dict(base, rope_scaling={"factor": 8.0, "low_freq_factor": 1.0}),
+            {k: v for k, v in base.items() if k not in ("num_key_value_heads", "rope_theta", "rope_scaling")},
+            dict({k: v for k, v in base.items() if k != "rope_theta"}, rotary_base=12345), dict(base, rope_scaling=2.0)]
+    cases = []
+    for c in cfgs:
+        ref = LlamaModelConfig(c)
+        cases.append({"config": c, "attrs": vars(ref),
+                      "kvslot_size": {"float16": ref.get_kvslot_size(torch.float16),
+                                      "bfloat16": ref.get_kvslot_size(torch.bfloat16)}})
+    save("model_config", cases=np.asarray(json.dumps(cases)))
+
+
+GENERATORS = {"elementwise": gen_elementwise, "kvcache_and_paged": gen_kvcache_and_paged, "prefill": gen_prefill,
+              "block_mgmt": gen_block_mgmt, "model": gen_model, "model_config": gen_model_config}
+
+
+def main(names):
+    """`names`: generators to run (all when empty), e.g. `python oracle/gen_golden.py model_config`."""
     os.makedirs(GOLDEN, exist_ok=True)
     swiftllm = ref_shim.import_reference()
-    gen_elementwise(swiftllm)
-    gen_kvcache_and_paged(swiftllm)
-    gen_prefill(swiftllm)
-    gen_block_mgmt(swiftllm)
-    gen_model(swiftllm)
+    for name in names or GENERATORS:
+        GENERATORS[name](swiftllm)
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])

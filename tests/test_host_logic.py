@@ -76,8 +76,9 @@ def test_fused_qkv_weight_views_share_storage():
     assert torch.equal(w1.up_gate_proj, torch.cat([w.up_gate_proj[256:512], w.up_gate_proj[512 + 256:]]))
 
 
-def test_bench_line_contract_helpers():
-    """bench.py helpers that run without a GPU: the workload description and the thread cap of the CPU arm."""
+def test_bench_line_contract_helpers(tmp_path):
+    """bench.py helpers that run without a GPU: the workload description, the thread cap of the CPU arm and the files of
+    --dump-outputs (the same column sample every run, within 64 MB at the flagship shape)."""
     import importlib.util, os, types
     spec = importlib.util.spec_from_file_location("bench", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
     bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
@@ -86,26 +87,28 @@ def test_bench_line_contract_helpers():
     assert cfg["global_batch"] == 256 and cfg["seq_len"] == 4096 and cfg["parallelism"] == "tp2" and "workload" in cfg
     assert 1 <= bench.cpu_threads() <= 32
     assert bench.METRIC == "decode_tokens_per_s" and bench.UNIT == "tokens/s"
+    B, V = 256, 128256
+    logits = torch.arange(V, dtype=torch.float32).expand(B, V)             # each logit holds its column index
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), torch.arange(B), logits)
+    tok, a, b = (np.load(tmp_path / p) for p in ("a/tokens.npy", "a/logits_sample.npy", "b/logits_sample.npy"))
+    assert tok.dtype == np.float64 and np.array_equal(tok, np.arange(B))
+    assert a.dtype == np.float32 and a.shape == (B, bench.DUMP_LOGIT_COLUMNS) and np.array_equal(a, b)
+    assert (np.diff(a[0]) > 0).all() and (a == a[0]).all()                  # distinct columns, the same for every sequence
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    bench.dump_outputs(str(tmp_path / "c"), torch.arange(B), None)          # sharded lm_head: tokens only
+    assert os.listdir(tmp_path / "c") == ["tokens.npy"]
 
 
-def test_model_config_matches_the_reference_parser_when_the_reference_is_mounted():
-    """Build-container only (skipped elsewhere): the unmodified reference's LlamaModelConfig and ours expose the same values for
-    every attribute the reference defines, over GQA / MHA / scaled-RoPE / legacy-key configs."""
-    import importlib.util
-    import os
-    import pytest
-    path = "/root/reference/swiftllm/model_config.py"
-    if not os.path.exists(path):
-        pytest.skip("reference tree not mounted")
-    spec = importlib.util.spec_from_file_location("ref_model_config", path)
-    ref = importlib.util.module_from_spec(spec); spec.loader.exec_module(ref)
-    base = dict(LLAMA3_8B)
-    cfgs = [base, dict(base, rope_scaling={"factor": 8.0, "low_freq_factor": 1.0}),
-            {k: v for k, v in base.items() if k not in ("num_key_value_heads", "rope_theta", "rope_scaling")},
-            dict({k: v for k, v in base.items() if k != "rope_theta"}, rotary_base=12345), dict(base, rope_scaling=2.0)]
-    for c in cfgs:
-        ours, theirs = LlamaModelConfig(c), ref.LlamaModelConfig(c)
-        for name, value in vars(theirs).items():
+def test_model_config_matches_the_reference_parser(golden):
+    """The unmodified reference's LlamaModelConfig (recorded in tests/golden/model_config.npz by oracle/gen_golden.py) and ours
+    expose the same values for every attribute the reference defines, over GQA / MHA / scaled-RoPE / legacy-key configs."""
+    import json
+    cases = json.loads(str(golden("model_config")["cases"]))
+    assert len(cases) == 5
+    for case in cases:
+        ours = LlamaModelConfig(case["config"])
+        for name, value in case["attrs"].items():
             assert getattr(ours, name) == value, name
-        for dt in (torch.float16, torch.bfloat16):
-            assert ours.get_kvslot_size(dt) == theirs.get_kvslot_size(dt)
+        for key, dt in (("float16", torch.float16), ("bfloat16", torch.bfloat16)):
+            assert ours.get_kvslot_size(dt) == case["kvslot_size"][key]
